@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ESRGAN 4x G/D training-step throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-cudnn]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-cudnn] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): RRDBNet 23 blocks nf=64 + VGG19-conv5_4 perceptual loss +
 Discriminator_VGG(256) vanilla RaGAN, 16 images / GPU, LR 64x64 -> HR 256x256, bf16 compute with
@@ -15,6 +15,9 @@ region, loss read back every step); roofline = tensor-pipe roofline of the domin
 cpu_baseline = the unmodified reference SRModel (baseline/_ref) on this box's host cores (bounded sample);
 vs_cudnn = the unmodified reference SRModel on this GPU through PyTorch/cuDNN (bf16 autocast and native fp16 AMP).
 --impl reference / reference-cudnn run ONLY the reference (they never import trainner_b200 or oracle/).
+cpu_baseline and vs_cudnn are null when no reference tree is staged (tools/stage_reference.py).
+--dump-outputs DIR writes what the last timed step computed (SR batch, losses, updated weights) as .npy files;
+the inputs are seeded, so runs with the same arguments on two builds can be compared output for output.
 """
 import argparse
 import contextlib
@@ -46,6 +49,8 @@ def parse():
     ap.add_argument("--hr", type=int, default=256)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cudnn-ref", action="store_true", help="skip the in-run reference-cuDNN rows (vs_cudnn)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -149,6 +154,33 @@ def timed_steps(fn, steps, warmup, world):
         dist.barrier()
         ms = float(t.item())
     return ms / steps
+
+
+DUMP_MAX_ELEMENTS = 4 << 20   # per array (16 MiB of float32): the dump stays under 64 MiB at any batch size
+
+
+def dump_outputs(model, out_dir):
+    """Write what a caller of the timed step holds after its last step, so that two builds can be compared output
+    for output: sr.npy (fake_H, float32), loss_<name>.npy (each log_dict value, float64) and netG_state.npy /
+    netD_state.npy (every floating-point state_dict tensor after the optimizer step, flattened and concatenated in
+    key order, float32).  An array of more than DUMP_MAX_ELEMENTS elements is replaced by the elements at a fixed
+    seeded sample of its flattened positions, the same positions in every run with the same arguments."""
+    import numpy as np
+    model.synchronize()
+    torch.cuda.synchronize()
+    arrays = [("sr", model.fake_H.detach().float())]
+    arrays += [("loss_" + k, torch.tensor(v, dtype=torch.float64)) for k, v in model.get_current_log().items()]
+    for name, net in (("netG", model.netG), ("netD", model.netD)):
+        if net is not None:
+            arrays.append((name + "_state", torch.cat([v.detach().float().flatten() for v in net.state_dict().values()
+                                                       if v.is_floating_point()])))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays:
+        a = a.cpu()
+        if a.numel() > DUMP_MAX_ELEMENTS:
+            pick = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMENTS]
+            a = a.flatten()[pick.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def reference_batch(args, batch, device=None, seed=1234):
@@ -273,11 +305,13 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
-    torch.manual_seed(0)
     vgg_path = vgg_checkpoint() if rank == 0 or world == 1 else None
     if world > 1:
         dist.barrier()
         vgg_path = vgg_checkpoint()
+    # seeded after vgg_checkpoint(), which draws from the global generator only when its cached file is missing:
+    # the initial weights are the same whether or not an earlier run left that file behind
+    torch.manual_seed(0)
     model = create_model(make_opt(args, vgg_path), device="cuda")
     gen = torch.Generator().manual_seed(1234 + rank)
     host = {"LR": torch.rand(args.batch, 3, args.hr // 4, args.hr // 4, generator=gen).pin_memory(),
@@ -303,6 +337,8 @@ def main():
     args.warmup = max(args.warmup, 4)
     sampler = ClockSampler(local) if rank == 0 else None
     ms = timed_steps(step_resident, args.steps, args.warmup, world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(model, args.dump_outputs)
     ms_e2e = timed_steps(step_e2e, args.steps, max(1, args.warmup // 2), world)
     clocks = sampler.stop() if sampler else None
 
@@ -370,13 +406,19 @@ def main():
                 "step_frac_of_peak": (GFLOP_PER_IMAGE_STEP * 1e9 * (args.batch / (ms / 1e3))) / (peak * 1e12),
                 "step_executed_tflops": (GFLOP_PER_IMAGE_STEP - 2 * 2 * 9.123) * 1e-3 * args.batch,
                 "step_frac_of_peak_executed": ((GFLOP_PER_IMAGE_STEP - 2 * 2 * 9.123) * 1e9 * (args.batch / (ms / 1e3))) / (peak * 1e12)}
-        if not args.no_cpu_baseline and world == 1 and rank == 0:
+        from baseline import reference_arm as RA
+        # the reference rows run the unmodified reference, which is not part of this repository: only where a
+        # reference tree has been staged (tools/stage_reference.py)
+        have_ref = RA.reference_available()
+        if not have_ref and world == 1 and rank == 0 and not (args.no_cpu_baseline and args.no_cudnn_ref):
+            print("bench: no reference tree staged; cpu_baseline and vs_cudnn are not measured", file=sys.stderr)
+        if have_ref and not args.no_cpu_baseline and world == 1 and rank == 0:
             c_ips, c_dt, threads = cpu_reference_steps(args, 6, 1)
             cpu_base = {"value": c_ips * px, "unit": "HR-px/s", "images_per_sec": c_ips, "cores": threads,
                         "kind": "reference",
                         "sample": "unmodified reference SRModel on CPU, 6 timed steps after 1 warm-up at 1 image per step "
                                   "(bounded sample of the %d-image step; nb=%d, HR %d^2), fp32" % (args.batch, args.nb, args.hr)}
-        if not args.no_cudnn_ref and world == 1 and rank == 0:
+        if have_ref and not args.no_cudnn_ref and world == 1 and rank == 0:
             # the reference's own GPU path on THIS B200, same config: the >= 6x target of BASELINE.json is
             # images/s of this repo over these rows (>= 20 warm-ups, >= 50 timed iterations each)
             vs_cudnn = {}

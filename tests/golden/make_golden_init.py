@@ -5,6 +5,7 @@ The B200 modules must consume the RNG in exactly the same order (module iteratio
 matching on 'Conv'/'Linear'/'BatchNorm2d', tensor shapes), so the same seed must give bit-identical tensors.
 Run in the build container only (needs /root/reference):  python tests/golden/make_golden_init.py
 """
+import math
 import os
 import sys
 from collections import OrderedDict
@@ -19,7 +20,9 @@ import torch  # noqa: E402
 
 
 def checksums(sd):
-    return OrderedDict((k, (float(v.double().sum()), float(v.double().abs().sum()))) for k, v in sd.items())
+    """exactly rounded sums (math.fsum): independent of how a reduction is split across threads or vector lanes"""
+    return OrderedDict((k, (math.fsum(v.double().flatten().tolist()), math.fsum(v.double().abs().flatten().tolist())))
+                       for k, v in sd.items())
 
 
 def main():

@@ -2,6 +2,7 @@
 nn.Module surface (state_dict keys/shapes, init) matches the reference's as recorded in the golden
 fixtures; the product path refuses to run without a GPU (no CPU fallback)."""
 import ctypes
+import math
 import os
 import re
 
@@ -122,7 +123,10 @@ def test_init_weights_bit_identical_to_reference():
     fx = torch.load(os.path.join(GOLD, "init.pt"))
 
     def checks(sd):
-        return [(k, (float(v.double().sum()), float(v.double().abs().sum()))) for k, v in sd.items()]
+        # exactly rounded sums (as make_golden_init.py records them): a float64 torch.sum splits its reduction by
+        # thread count, which moves the last bit from one machine to the next
+        return [(k, (math.fsum(v.double().flatten().tolist()), math.fsum(v.double().abs().flatten().tolist())))
+                for k, v in sd.items()]
 
     for mode in ("upconv", "pixelshuffle"):
         torch.manual_seed(1234)
@@ -152,27 +156,3 @@ def test_product_code_never_imports_oracle():
             if f.endswith(".py") or f.endswith(".cu") or f.endswith(".cuh"):
                 src = open(os.path.join(dirpath, f)).read()
                 assert "import oracle" not in src and "from oracle" not in src, f
-
-
-def test_bench_reference_arm_json_contract():
-    """`bench.py --impl reference` (the UNMODIFIED reference SRModel from baseline/_ref, timed on host cores) prints
-    ONE JSON line with the keys the driver reads and loads neither trainner_b200 nor oracle/; tiny configuration so
-    that it runs in seconds."""
-    from baseline import reference_arm
-    if not reference_arm.reference_available():
-        pytest.skip("reference tree not staged (tools/stage_reference.py)")
-    import json
-    import subprocess
-    import sys
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--nb", "1",
-                          "--hr", "32", "--steps", "1", "--warmup", "1"], capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0, out.stderr[-2000:]
-    line = json.loads(out.stdout.strip().splitlines()[-1])
-    assert line["impl"] == "reference" and line["metric"] == "hr_pixels_per_sec" and line["unit"] == "HR-px/s"
-    assert line["higher_is_better"] is True and line["n_gpus"] == 1 and line["steps"] == 1 and line["value"] > 0
-    assert len(out.stdout.strip().splitlines()) == 1, out.stdout
-    assert line["cpu_baseline"]["kind"] == "reference" and line["cpu_baseline"]["cores"] >= 1
-    assert line["loaded"] == {"trainner_b200": False, "oracle": False}
-    assert line["cpu_baseline"]["value"] == line["value"]
-    assert line["e2e"]["value"] == line["value"] and line["e2e"]["h2d_bytes_per_step"] == 0 \
-        and line["e2e"]["d2h_bytes_per_step"] == 0
