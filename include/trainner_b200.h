@@ -69,7 +69,7 @@ int b200_conv_igemm(const b200_conv_desc* d, const void* x, const void* w_packed
                     b200_stream_t stream);
 /* The same conv (no residual / mask / activation operands) that ALSO writes the BatchNorm partial statistics of
  * its bf16-rounded output from the epilogue: stat_part is fp32 [2][cout][rows], rows = b200_conv_igemm_stat_rows(d)
- * (0 when this shape is not served by the statistics epilogue -- use b200_bn_stats then; < 0 on error).
+ * (0 when this shape is not served by the statistics epilogue -- use b200_bn_stats_finalize then; < 0 on error).
  * Replaces the separate pass of nn.BatchNorm2d's batch statistics over the conv output (block.py:122).        */
 int b200_conv_igemm_stat_rows(const b200_conv_desc* d);
 int b200_conv_igemm_stats(const b200_conv_desc* d, const void* x, const void* w_packed, const float* bias,
@@ -116,39 +116,13 @@ int b200_unpad_add(void* dst_dense, int32_t dst_c, const void* src_flat, int32_t
                    const void* add_dense, int32_t add_c, int32_t n, int32_t h, int32_t w, int32_t c,
                    b200_stream_t stream);
 
-/* TMEM-persistent, stage-merged residual dense block (csrc/rdb_persist.cu): one launch computes the
- * whole block -- forward, or its input gradient in gather form.  Stage j consumes one 64/32-channel
- * input slice and accumulates into all not-yet-complete output columns (192 - 32 j of them, fp32 in
- * TMEM for the whole block); the 32 (last stage 64) columns completed by stage j are finished with
- * the stage's epilogue and written to `out`, which is the next stage's input.
- * w_packed: bf16 [9 taps][192 - 32 j rows][64 cols] (b200_pack_cat).  All tensors flat
- * [n, h+2, w+2, c]; n*(h+2)*(w+2) <= 256 * #SMs (one tile per CTA, cooperative launch).
- * flags: zero-initialised int array of >= #tiles; flag_base must grow by >= 8 per launch.       */
-typedef struct {
-  const void* x; int32_t cx, cin_off, cin;       /* input slice (cin = 64 or 32)                */
-  const void* w_packed;
-  void* out; int32_t out_c, out_coff;             /* completing slice                            */
-  const float* bias;                              /* [32] ([64] for the last stage) or NULL     */
-  const void* mask; int32_t mask_c, mask_coff;    /* v *= lrelu'(mask) with mask_slope          */
-  const void* res1; int32_t res1_c, res1_coff;
-  const void* res2; int32_t res2_c, res2_coff;
-  float alpha, beta1, beta2, slope, mask_slope;   /* v = alpha*(acc+bias) + beta1*res1 + beta2*res2 -> lrelu(slope) if act */
-  int32_t act;
-} b200_rdb_stage;
-
-typedef struct {
-  int32_t n, h, w;
-  int32_t flip_taps;   /* 0: input offset of weight tap (ky,kx) is (ky-1, kx-1) (forward); 1: (1-ky, 1-kx) (input gradient) */
-  b200_rdb_stage stage[5];
-} b200_rdb_desc;
-
-int b200_rdb_persist(const b200_rdb_desc* d, int32_t* flags, int32_t flag_base, b200_stream_t stream);
-
-/* Whole-trunk chain of dense blocks in ONE persistent launch (csrc/rdb_chain.cu): the stage-merged form of
- * b200_rdb_persist with the finished slices kept in shared memory as the next stage's operand, two independent
- * 128-position tiles per CTA and the halo rows exchanged through L2 in flag-in-data (LL) form.  Replaces the
- * 5 x n_blocks per-conv launches of ResidualDenseBlock_5C.forward / RRDB.forward (RRDBNet_arch.py:89-96,150-163)
- * and of their input gradients.  Stage s = 5*block + j: input slice = the output slice of stage s-1 (stage 0:
+/* Whole-trunk chain of dense blocks in ONE persistent launch (csrc/rdb_chain.cu).  A block is computed input
+ * slice by input slice: stage j adds the newest slice's contribution to every conv that still needs it, with the
+ * fp32 partial sums of a CTA's 256-position super-tile kept in TMEM for the whole block, and the slice each stage
+ * completes is kept in shared memory as the next stage's operand.  One CTA per super-tile, all co-resident; halo
+ * rows travel between neighbouring CTAs of a thread-block cluster through distributed shared memory and across
+ * cluster edges through L2 in flag-in-data (LL) form.  Replaces the 5 x n_blocks per-conv launches of
+ * ResidualDenseBlock_5C.forward / RRDB.forward (RRDBNet_arch.py:89-96,150-163) and of their input gradients.  Stage s = 5*block + j: input slice = the output slice of stage s-1 (stage 0:
  * channels [x_coff, x_coff+64) of x0), epilogue
  *   v = alpha*(acc + bias) + beta1*res1 + beta2*res2 ; act ? lrelu(v, slope) ; mask ? (mask > 0 ? v : mask_slope*v)
  * for the 32 (j = 4: 64) channels that stage completes, stored to out[m*out_c + out_coff ..] (bf16, interior
@@ -173,7 +147,8 @@ typedef struct {
   int32_t flip_taps;          /* 0: forward taps; 1: input-gradient taps */
 } b200_chain_desc;
 
-/* CTAs (= co-resident tile pairs; must not exceed the SM count) and exchange-buffer bytes for n images */
+/* CTAs (= 256-position super-tiles; must not exceed the SM count) and exchange-buffer bytes for n images;
+ * returns nonzero when the image is too wide for the kernel (w > 125) */
 int b200_rdb_chain_geometry(int32_t n, int32_t h, int32_t w, int32_t* n_cta, int64_t* ll_bytes);
 /* w_stage[j]: packed stage weights [n_blocks][9][192-32j][K_j] bf16 (K_0 = 64, K_j = 32); table_dev:
  * [n_blocks][5] b200_chain_stage in device memory; ll_buf: zero-initialised once, reused by every launch;
@@ -282,18 +257,15 @@ int b200_conv3x3_thin_wgrad(const float* thin, const void* wide, float* dw, floa
                             const float* mean, const float* std, b200_stream_t stream);
 
 /* BatchNorm2d (training mode, batch statistics) + LeakyReLU on NHWC bf16 -- block.py:122,91.
- * stats: fp32 [2][c] = sum, sumsq over n*h*w (zeroed by the call).                           */
-int b200_bn_stats(const void* z, float* stats, int64_t npix, int32_t c, b200_stream_t stream);
-int b200_bn_finalize(const float* stats, float* mean_invstd, float* running_mean,
-                     float* running_var, int64_t npix, int32_t c, float momentum, float eps,
-                     b200_stream_t stream);
-/* b200_bn_stats + b200_bn_finalize in one launch: the block that produces the totals also writes mean / invstd
- * and updates the running statistics (the default training-mode forward; nn.BatchNorm2d semantics).          */
+ * b200_bn_stats_finalize: stats = fp32 [2][c] sum, sumsq over n*h*w (zeroed by the call); the block that produces
+ * the totals also writes mean_invstd = [2][c] mean, invstd and updates the running statistics (when non-null) in
+ * the same launch (nn.BatchNorm2d semantics).                                                                    */
 int b200_bn_stats_finalize(const void* z, float* stats, float* mean_invstd, float* running_mean,
                            float* running_var, int64_t npix, int32_t c, float momentum, float eps,
                            b200_stream_t stream);
-/* b200_bn_finalize for many layers in one launch (the running-statistics side effect of a re-used train-mode
- * forward: 11 layers x 2 re-used forwards per step).  table: device array of b200_bn_finalize_entry.            */
+/* The finishing step of b200_bn_stats_finalize (stats -> mean_invstd + running statistics) for many layers in
+ * one launch (the running-statistics side effect of a re-used train-mode forward: 11 layers x 2 re-used forwards
+ * per step).  table: device array of b200_bn_finalize_entry.                                                    */
 typedef struct {
   const float* stats;   /* [2][c] sum, sum of squares */
   float* mean_invstd;   /* [2][c] */
@@ -308,7 +280,7 @@ int b200_bn_finalize_multi(const b200_bn_finalize_entry* table_dev, int32_t coun
                            b200_stream_t stream);
 /* BatchNorm statistics from the conv epilogue instead of a pass over z: b200_conv_igemm_stats (below) writes one
  * row of per-channel (sum, sum of squares) per 128-pixel half tile into part[2][c][rows]; this adds the rows in a
- * fixed order and finishes like b200_bn_finalize.  rows = b200_conv_igemm_stat_rows(desc).                      */
+ * fixed order and finishes like b200_bn_stats_finalize.  rows = b200_conv_igemm_stat_rows(desc).                */
 int b200_bn_partials_finalize(const float* part, int32_t rows, float* stats, float* mean_invstd,
                               float* running_mean, float* running_var, int64_t npix, int32_t c, float momentum,
                               float eps, b200_stream_t stream);
@@ -343,9 +315,6 @@ int b200_pixel_shuffle2(const void* z, void* out, int32_t n, int32_t h, int32_t 
                         int32_t act, float slope, b200_stream_t stream);
 int b200_pixel_unshuffle2(const void* dout, void* dz, int32_t n, int32_t h, int32_t w, int32_t c,
                           b200_stream_t stream);
-/* dst[p, dst_coff + c] += src[p, src_coff + c] on NHWC bf16 slices                              */
-int b200_add_slice_bf16(void* dst, int32_t dst_c, int32_t dst_coff, const void* src, int32_t src_c,
-                        int32_t src_coff, int64_t npix, int32_t c, b200_stream_t stream);
 
 /* L1 loss (mean |a-b|) forward + gradient in one pass -- losses.py:37-39.
  * fp32 variant: a, b fp32, grad_a fp32 = gscale*sign(a-b)/numel.  bf16 variant likewise.
@@ -362,7 +331,6 @@ int b200_nchw_f32_to_nhwc_bf16(const float* x, void* y, int32_t n, int32_t c, in
                                int32_t cy, int32_t y_coff, b200_stream_t stream);
 int b200_nhwc_bf16_to_nchw_f32(const void* x, float* y, int32_t n, int32_t c, int32_t h, int32_t w,
                                int32_t cx, int32_t x_coff, b200_stream_t stream);
-int b200_add_f32(float* dst, const float* src, int64_t numel, b200_stream_t stream);
 
 const char* b200_last_error(void);
 int b200_version(void);

@@ -342,13 +342,14 @@ def test_psnr_after_training_matches_reference_paths():
     assert abs(mb - m32) <= max(1.5, 2.0 * abs(m16 - m32)), (m32, m16, mb)
 
 
-@pytest.mark.parametrize("shape", [(3, 12, 20, 2), (2, 16, 16, 1), (16, 64, 64, 23)])
+@pytest.mark.parametrize("shape", [(3, 12, 20, 2), (2, 16, 16, 1), (16, 64, 64, 23), (2, 24, 96, 2)])
 def test_trunk_chain_matches_per_conv_flat_path(shape, monkeypatch):
     """The whole-trunk chain kernel (csrc/rdb_chain.cu: stage-merged dense blocks, TMEM-resident partial sums,
     slices turned around in shared memory, LL halo exchange) against the per-conv flat kernels (conv_flat.cu) on
     the same weights: both store every slice in bf16 and accumulate in fp32, only the summation order differs.
-    Covers an odd image count (unequal position ranges), a single-tile-per-range case and BASELINE config 2's
-    trunk at its real size (nb = 23, 16 x 64 x 64: two launches of 8 images, 137 CTAs)."""
+    Covers an odd image count (unequal position ranges), a single-tile-per-range case, BASELINE config 2's
+    trunk at its real size (nb = 23, 16 x 64 x 64: two launches of 8 images, 137 CTAs) and a 96-wide image, where
+    three operand regions do not fit and the chain issues every stage in one piece with two regions (20 CTAs)."""
     from trainner_b200 import networks
     from trainner_b200.architectures import RRDBNet_arch
     n, h, w, nb = shape
@@ -368,6 +369,9 @@ def test_trunk_chain_matches_per_conv_flat_path(shape, monkeypatch):
             y.backward(torch.ones_like(y) * 0.5 if rep else torch.sign(y.detach() - 0.1))
         eng = net._engine[0]
         assert eng.chain == (chain == "1")
+        ctx = eng.pools[(n, h, w)].all[0]
+        tags = {m[0] for m in ctx.fwd.meta + ctx.bwd.meta}
+        assert ("rdb_chain" in tags) == (chain == "1"), tags   # the plans, not just the engine, took the chain
         outs.append(y.detach().float())
         grads.append(OrderedDict((k, p.grad.detach().float().clone()) for k, p in net.named_parameters()))
     e = rel(outs[1], outs[0])

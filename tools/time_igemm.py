@@ -1,5 +1,5 @@
 """Per-layer timing of the implicit-GEMM conv (csrc/conv_igemm.cu) at config-2 shapes.
-    python tools/time_igemm.py            # B200_IGEMM_PATCH=0/1, B200_IGEMM_DEBUG=1 are honoured by the library
+    python tools/time_igemm.py            # B200_IGEMM_DEBUG=1 is honoured by the library
 """
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -88,23 +88,6 @@ class PackCatEntry(C.Structure):
                 ("scale", C.c_float), ("row_off", C.c_int32), ("mode", C.c_int32), ("pad_", C.c_int32)]
 
 
-class RdbStage(C.Structure):
-    _fields_ = [("x", C.c_void_p), ("cx", C.c_int32), ("cin_off", C.c_int32), ("cin", C.c_int32),
-                ("w_packed", C.c_void_p),
-                ("out", C.c_void_p), ("out_c", C.c_int32), ("out_coff", C.c_int32),
-                ("bias", C.c_void_p),
-                ("mask", C.c_void_p), ("mask_c", C.c_int32), ("mask_coff", C.c_int32),
-                ("res1", C.c_void_p), ("res1_c", C.c_int32), ("res1_coff", C.c_int32),
-                ("res2", C.c_void_p), ("res2_c", C.c_int32), ("res2_coff", C.c_int32),
-                ("alpha", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float), ("slope", C.c_float),
-                ("mask_slope", C.c_float), ("act", C.c_int32)]
-
-
-class RdbDesc(C.Structure):
-    _fields_ = [("n", C.c_int32), ("h", C.c_int32), ("w", C.c_int32), ("flip_taps", C.c_int32),
-                ("stage", RdbStage * 5)]
-
-
 class ChainStage(C.Structure):
     _fields_ = [("out", C.c_void_p), ("bias", C.c_void_p), ("mask", C.c_void_p), ("res1", C.c_void_p),
                 ("res2", C.c_void_p),
@@ -135,7 +118,6 @@ _SIGNATURES = {
     "b200_conv_igemm_stats": [_P, _P, _P, _P, _P, _P, _P],
     "b200_conv3x3_flat": [C.POINTER(FlatDesc), _P, _P, _P, _P, _P, _P, _P, _P, _P],
     "b200_pack_cat": [_P, _I, _I, _P],
-    "b200_rdb_persist": [C.POINTER(RdbDesc), _P, _I, _P],
     "b200_rdb_chain": [C.POINTER(ChainDesc), _P, _P, _P, _P, _L, _P, _P],
     "b200_rdb_chain_geometry": [_I, _I, _I, _P, _P],
     "b200_pad_copy": [_P, _I, _I, _P, _I, _I, _I, _I, _I, _I, _P],
@@ -149,8 +131,6 @@ _SIGNATURES = {
                                   _P, _I, _I, _F, _P],
     "b200_conv3x3_wide_to_thin": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _F, _P],
     "b200_conv3x3_thin_wgrad": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P],
-    "b200_bn_stats": [_P, _P, _L, _I, _P],
-    "b200_bn_finalize": [_P, _P, _P, _P, _L, _I, _F, _F, _P],
     "b200_bn_stats_finalize": [_P, _P, _P, _P, _P, _L, _I, _F, _F, _P],
     "b200_bn_partials_finalize": [_P, _I, _P, _P, _P, _P, _L, _I, _F, _F, _P],
     "b200_bn_finalize_multi": [_P, _I, _I, _P],
@@ -162,13 +142,11 @@ _SIGNATURES = {
     "b200_sumpool2x2_mask": [_P, _P, _P, _I, _I, _I, _I, _F, _P],
     "b200_pixel_shuffle2": [_P, _P, _I, _I, _I, _I, _I, _F, _P],
     "b200_pixel_unshuffle2": [_P, _P, _I, _I, _I, _I, _P],
-    "b200_add_slice_bf16": [_P, _I, _I, _P, _I, _I, _L, _I, _P],
     "b200_l1_loss_f32": [_P, _P, _P, _P, _L, _F, _P],
     "b200_l1_loss_bf16": [_P, _P, _P, _P, _L, _F, _P],
     "b200_lrelu_mask_mul": [_P, _P, _P, _L, _F, _P],
     "b200_nchw_f32_to_nhwc_bf16": [_P, _P, _I, _I, _I, _I, _I, _I, _P],
     "b200_nhwc_bf16_to_nchw_f32": [_P, _P, _I, _I, _I, _I, _I, _I, _P],
-    "b200_add_f32": [_P, _P, _L, _P],
 }
 
 EXPORTED_SYMBOLS = sorted(list(_SIGNATURES) + ["b200_last_error", "b200_version", "b200_device_ok",

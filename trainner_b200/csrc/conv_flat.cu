@@ -11,8 +11,8 @@
 // L2->SMEM traffic per MMA drops ~4.4x vs per-tap loading (conv_igemm.cu), which is what bounds
 // the per-tap kernel on the Cout=32 / Cin=32 trunk layers.
 //
-// Warp roles as in conv_igemm.cu: warp 0 TMA producer (A ring + B ring), warp 1 MMA issuer,
-// warps 2..5 epilogue (only interior rows are stored; the border stays zero).
+// Warp roles: warp 0 TMA producer (A ring + B ring), warps 1-2 MMA issuers (one per 128-row half),
+// warps 3..10 epilogue (only interior rows are stored; the border stays zero).
 // Reference: ResidualDenseBlock_5C / RRDB forward and autograd dgrad (RRDBNet_arch.py:89-163).
 #include <stdlib.h>
 
@@ -43,7 +43,7 @@ struct FlatParams {
   int a_stages, b_stages;
   int tpb;             // taps per B stage (9, 3 or 1): one barrier round-trip per tpb taps
   uint32_t b_ring_off;
-  int BN, acc_cols, acc_stages, Cout, tmem_cols;
+  int BN, acc_cols, acc_stages, Cout;
   // output
   __nv_bfloat16* out;
   int out_mode, cy, o_coff;
@@ -216,13 +216,8 @@ __device__ __forceinline__ void flat_issue_chunk(const FlatParams& p, const uint
   }
 }
 
-// EW = number of epilogue warps.  EW = 8: one CTA per SM (all of shared memory, 2-deep activation ring,
-// each CTA walks 2 tiles).  EW = 4: half the shared memory, registers and TMEM per CTA so that TWO CTAs
-// are co-resident per SM -- one CTA's prologue, operand-load latency and epilogue then overlap the other
-// CTA's MMAs, and with programmatic dependent launch the next conv's CTAs are already resident and set
-// up while this conv drains.
-template <int EW>
-__global__ void __launch_bounds__(96 + 32 * EW, EW == 4 ? 2 : 1)
+// One CTA per SM (all of shared memory and TMEM); each CTA walks the tiles with stride gridDim.x.
+__global__ void __launch_bounds__(kThreads, 1)
 conv_flat_kernel(const __grid_constant__ FlatParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem =
@@ -245,8 +240,8 @@ conv_flat_kernel(const __grid_constant__ FlatParams p) {
     }
     mbar_init(&tfull_bar[0], 2);
     mbar_init(&tfull_bar[1], 2);
-    mbar_init(&tempty_bar[0], EW);
-    mbar_init(&tempty_bar[1], EW);
+    mbar_init(&tempty_bar[0], 8);   // all epilogue warps
+    mbar_init(&tempty_bar[1], 8);
     mbar_fence_init();
   }
   if (warp == 0 && lane == 0) {
@@ -255,7 +250,7 @@ conv_flat_kernel(const __grid_constant__ FlatParams p) {
     tma_prefetch_desc(&p.w_map);
   }
   if (warp == 1) {
-    tmem_alloc(&tmem_base_s, p.tmem_cols);
+    tmem_alloc(&tmem_base_s, 512);
     tmem_relinquish();
   }
   tc_fence_before();
@@ -363,53 +358,49 @@ conv_flat_kernel(const __grid_constant__ FlatParams p) {
       }
     }
   } else {
-    // ------------------------------------------------------------ epilogue (warps 3..3+EW-1)
-    // EW = 8: warps 3..6 -> rows [0,128), warps 7..10 -> rows [128,256); EW = 4: each warp does both halves.
+    // ------------------------------------------------------------ epilogue (warps 3..10)
+    // warps 3..6 -> rows [0,128), warps 7..10 -> rows [128,256)
     const int quad = warp & 3;            // TMEM lane quadrant accessible by this warp
-    constexpr int NH = (EW == 8) ? 1 : 2;
+    const int half = (warp - 3) >> 2;
     int acc = 0;
     uint32_t acc_phase = 0;
     for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
       mbar_wait(&tfull_bar[acc], acc_phase);
       tc_fence_after();
       if (warp == 3) DBG_T(tile == (int)blockIdx.x ? 5 : 7);
-#pragma unroll 1
-      for (int hh = 0; hh < NH; ++hh) {
-        const int half = (EW == 8) ? ((warp - 3) >> 2) : hh;
-        const long long m = (long long)tile * kTileM + half * 128 + quad * 32 + lane;
-        const int nimg = (int)(m / p.HpWp);
-        const int rem = (int)(m - (long long)nimg * p.HpWp);
-        const int yp = rem / p.Wp, xp = rem - yp * p.Wp;
-        const bool valid = (m < p.P) && yp >= 1 && yp <= p.h && xp >= 1 && xp <= p.w;
-        __nv_bfloat16* out_px;
-        long long up_sx = 0, up_sy = 0;
-        if (p.out_mode == 0) {
-          out_px = p.out + m * p.cy;
-        } else if (p.out_mode == 1) {
-          out_px = p.out + (((long long)nimg * p.h + (yp - 1)) * p.w + (xp - 1)) * p.cy;
-        } else {
-          up_sx = p.cy;
-          up_sy = (long long)2 * p.w * p.cy;
-          out_px = p.out + (((long long)nimg * 2 * p.h + 2 * (yp - 1)) * 2 * p.w + 2 * (xp - 1)) * p.cy;
-        }
-        const uint32_t t_row = tmem + ((uint32_t)(quad * 32) << 16) + acc * 2 * p.acc_cols + half * p.acc_cols;
-        int c0 = 0;
-        for (; c0 + 32 <= p.BN; c0 += 32) {
-          uint32_t r[32];
-          tmem_ld_32x32b_x32(t_row + c0, r);
-          EpiLoads<32> L;
-          if (valid) flat_epilogue_load<32>(p, L, c0, m, out_px);
-          tmem_ld_wait();
-          if (valid) flat_epilogue<32>(p, r, L, c0, out_px, up_sx, up_sy);
-        }
-        if (c0 < p.BN) {
-          uint32_t r[16];
-          tmem_ld_32x32b_x16(t_row + c0, r);
-          EpiLoads<16> L;
-          if (valid) flat_epilogue_load<16>(p, L, c0, m, out_px);
-          tmem_ld_wait();
-          if (valid) flat_epilogue<16>(p, r, L, c0, out_px, up_sx, up_sy);
-        }
+      const long long m = (long long)tile * kTileM + half * 128 + quad * 32 + lane;
+      const int nimg = (int)(m / p.HpWp);
+      const int rem = (int)(m - (long long)nimg * p.HpWp);
+      const int yp = rem / p.Wp, xp = rem - yp * p.Wp;
+      const bool valid = (m < p.P) && yp >= 1 && yp <= p.h && xp >= 1 && xp <= p.w;
+      __nv_bfloat16* out_px;
+      long long up_sx = 0, up_sy = 0;
+      if (p.out_mode == 0) {
+        out_px = p.out + m * p.cy;
+      } else if (p.out_mode == 1) {
+        out_px = p.out + (((long long)nimg * p.h + (yp - 1)) * p.w + (xp - 1)) * p.cy;
+      } else {
+        up_sx = p.cy;
+        up_sy = (long long)2 * p.w * p.cy;
+        out_px = p.out + (((long long)nimg * 2 * p.h + 2 * (yp - 1)) * 2 * p.w + 2 * (xp - 1)) * p.cy;
+      }
+      const uint32_t t_row = tmem + ((uint32_t)(quad * 32) << 16) + acc * 2 * p.acc_cols + half * p.acc_cols;
+      int c0 = 0;
+      for (; c0 + 32 <= p.BN; c0 += 32) {
+        uint32_t r[32];
+        tmem_ld_32x32b_x32(t_row + c0, r);
+        EpiLoads<32> L;
+        if (valid) flat_epilogue_load<32>(p, L, c0, m, out_px);
+        tmem_ld_wait();
+        if (valid) flat_epilogue<32>(p, r, L, c0, out_px, up_sx, up_sy);
+      }
+      if (c0 < p.BN) {
+        uint32_t r[16];
+        tmem_ld_32x32b_x16(t_row + c0, r);
+        EpiLoads<16> L;
+        if (valid) flat_epilogue_load<16>(p, L, c0, m, out_px);
+        tmem_ld_wait();
+        if (valid) flat_epilogue<16>(p, r, L, c0, out_px, up_sx, up_sy);
       }
       tc_fence_before();
       __syncwarp();
@@ -426,7 +417,7 @@ conv_flat_kernel(const __grid_constant__ FlatParams p) {
   tc_fence_before();
   __syncthreads();
   if (warp == 0) DBG_T(9);
-  if (warp == 1) tmem_dealloc(tmem, p.tmem_cols);
+  if (warp == 1) tmem_dealloc(tmem, 512);
 }
 
 // ---------------------------------------------------------------- layout helpers
@@ -498,15 +489,8 @@ extern "C" int b200_conv3x3_flat(const b200_flat_desc* d, const void* x, const v
   B200_REQUIRE(d->cout > 0 && d->cout % 16 == 0 && d->cout <= 192, "b200_conv3x3_flat: cout %% 16, <= 192");
   B200_REQUIRE(d->cx % 8 == 0 && d->cy % 8 == 0 && d->cin_off % 8 == 0 && d->cout_off % 8 == 0,
                "b200_conv3x3_flat: channel pitches/offsets must be multiples of 8");
-  static int two_cta = -1;   // measured slower at ~1.85 tiles per SM (both CTAs run in lockstep); opt-in via B200_FLAT_2CTA=1
   const int kSmemBytes = 200 * 1024;
-  const int kSmemBytes2 = 112 * 1024;   // two co-resident CTAs per SM (228 KB - 1 KB reserved per CTA)
-  B200_ENSURE_SMEM(conv_flat_kernel<8>, kSmemBytes);
-  if (::b200::ensure_max_smem(reinterpret_cast<const void*>(conv_flat_kernel<4>), kSmemBytes2, true)) return 1;
-  if (two_cta < 0) {
-    const char* e = getenv("B200_FLAT_2CTA");
-    two_cta = e ? atoi(e) : 0;
-  }
+  B200_ENSURE_SMEM(conv_flat_kernel, kSmemBytes);
   FlatParams p;
   memset(&p, 0, sizeof(p));
   p.n = d->n; p.h = d->h; p.w = d->w;
@@ -546,28 +530,7 @@ extern "C" int b200_conv3x3_flat(const b200_flat_desc* d, const void* x, const v
   // taps per B stage: fewer barrier round trips for the MMA issuers when the weight tiles are small
   p.tpb = (9 * p.b_tap_bytes <= 40 * 1024) ? 9 : ((3 * p.b_tap_bytes <= 50 * 1024) ? 3 : 1);
   p.b_stage_bytes = p.b_tap_bytes * p.tpb;
-  p.tmem_cols = 512;
-  bool use2 = false;
-  if (two_cta && 2 * p.acc_cols * p.acc_stages <= 256) {
-    // half-SM configuration: one activation stage, >= 2 weight stages of as many taps as fit
-    const int budget2 = kSmemBytes2 - 2048 - (int)p.a_stage_bytes;
-    for (int tpb : {9, 3, 1}) {
-      const int st = (int)p.b_tap_bytes * tpb;
-      if (budget2 >= 2 * st) {
-        use2 = true;
-        p.tpb = tpb;
-        p.b_stage_bytes = (uint32_t)st;
-        p.a_stages = 1;
-        p.b_stages = budget2 / st;
-        if (p.b_stages > kMaxBStages) p.b_stages = kMaxBStages;
-        int need = 2 * p.acc_cols * p.acc_stages;
-        p.tmem_cols = 32;
-        while (p.tmem_cols < need) p.tmem_cols *= 2;
-        break;
-      }
-    }
-  }
-  if (!use2) {
+  {
     // Shared-memory fit: prefer 2-3 activation stages and the largest weight stage (fewest barrier round
     // trips); wide images (large A region: (256 + 2(w+3)) rows x 128 B per stage) fall back to fewer taps
     // per weight stage and finally to a single activation stage.  Widest LR input that fits: w ~ 580.
@@ -644,13 +607,8 @@ extern "C" int b200_conv3x3_flat(const b200_flat_desc* d, const void* x, const v
   }
   const int sms = sm_count();
   const size_t smem = (size_t)p.a_stages * p.a_stage_bytes + (size_t)p.b_stages * p.b_stage_bytes + 1024;
-  if (use2) {
-    const int grid = p.total_tiles < 2 * sms ? p.total_tiles : 2 * sms;
-    ::b200::launch_kernel(conv_flat_kernel<4>, grid, 96 + 32 * 4, smem, as_stream(stream), p);
-  } else {
-    const int grid = p.total_tiles < sms ? p.total_tiles : sms;
-    ::b200::launch_kernel(conv_flat_kernel<8>, grid, kThreads, smem, as_stream(stream), p);
-  }
+  const int grid = p.total_tiles < sms ? p.total_tiles : sms;
+  ::b200::launch_kernel(conv_flat_kernel, grid, kThreads, smem, as_stream(stream), p);
   B200_LAUNCH_CHECK();
   return 0;
 }

@@ -733,7 +733,8 @@ inline int pow2_ceil(int v) {
 using namespace b200;
 
 // stat_part != nullptr: also produce the BatchNorm partial statistics (EPI = 3); stat_query != nullptr: launch
-// nothing, only report how many partial rows that would produce (0 = this conv cannot: fall back to b200_bn_stats).
+// nothing, only report how many partial rows that would produce (0 = this conv cannot: fall back to
+// b200_bn_stats_finalize).
 static int conv_igemm_impl(const b200_conv_desc* d, const void* x, const void* w_packed, const float* bias,
                            const void* res1, const void* res2, const void* mask, void* y, float* stat_part,
                            int* stat_query, b200_stream_t stream) {
@@ -847,11 +848,7 @@ static int conv_igemm_impl(const b200_conv_desc* d, const void* x, const void* w
   p.dbg_ptr = igemm_dbg_ptr;
   // straight-line epilogue with staged TMA tile stores (conv_igemm256_kernel<1 / 2>): whole 64-channel slabs, no
   // residual / accumulate operands
-  static const bool fast_epi_enabled = [] {
-    const char* e = getenv("B200_IGEMM_FAST_EPI");
-    return !(e && e[0] == '0');
-  }();
-  p.tma_store = use256 && fast_epi_enabled && BN % 64 == 0 && !res1 && !res2 && !d->accumulate;
+  p.tma_store = use256 && BN % 64 == 0 && !res1 && !res2 && !d->accumulate;
   if (p.tma_store) {
     const int kSlab = 128 * 128;   // one half's 64-channel slab
     p.st_bufs = 2;

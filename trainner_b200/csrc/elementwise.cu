@@ -153,21 +153,11 @@ __global__ void bn_reduce_kernel(const __nv_bfloat16* __restrict__ z,
   });
   if (MODE == 0 && fin && fin_mean_invstd) {
     // the block that produced the totals also turns them into mean / invstd and the running statistics
-    // (same arithmetic as bn_finalize_kernel): one launch less per BatchNorm layer
+    // (bn_finalize_channel, as in the other finalize kernels): one launch less per BatchNorm layer
     __syncthreads();
     for (int ch = threadIdx.x; ch < c; ch += blockDim.x)
       bn_finalize_channel(sums, fin_mean_invstd, running_mean, running_var, npix, c, momentum, eps, ch);
   }
-}
-
-__global__ void bn_finalize_kernel(const float* __restrict__ stats, float* __restrict__ mean_invstd,
-                                   float* __restrict__ running_mean, float* __restrict__ running_var,
-                                   long long npix, int c, float momentum, float eps) {
-  pdl_trigger();
-  pdl_wait();
-  const int ch = blockIdx.x * blockDim.x + threadIdx.x;
-  if (ch >= c) return;
-  bn_finalize_channel(stats, mean_invstd, running_mean, running_var, npix, c, momentum, eps, ch);
 }
 
 __global__ void bn_finalize_multi_kernel(const b200_bn_finalize_entry* __restrict__ table) {
@@ -181,7 +171,7 @@ __global__ void bn_finalize_multi_kernel(const b200_bn_finalize_entry* __restric
 
 // BatchNorm statistics from the per-tile partial sums the conv epilogue wrote (conv_igemm EPI = 3; output-major
 // part[(which * c + ch) * rows + r]): one warp per channel adds the rows in a fixed order (lane-strided, then a
-// butterfly), so the result is deterministic, then finishes the channel like bn_finalize_kernel.
+// butterfly), so the result is deterministic, then finishes the channel with bn_finalize_channel.
 __global__ void __launch_bounds__(256) bn_partials_finalize_kernel(const float* __restrict__ part, int rows,
                                                                    float* __restrict__ stats,
                                                                    float* __restrict__ mean_invstd,
@@ -530,34 +520,6 @@ __global__ void nhwc_to_nchw_kernel(const __nv_bfloat16* __restrict__ x, float* 
     y[i] = __bfloat162float(x[(b * h * w + hw) * cx + coff + ch]);
   }
 }
-__global__ void add_slice_kernel(__nv_bfloat16* __restrict__ dst, int dst_c, int dst_coff,
-                                 const __nv_bfloat16* __restrict__ src, int src_c, int src_coff,
-                                 long long npix, int c) {
-  pdl_trigger();
-  pdl_wait();
-  const int cv = c / 8;
-  const long long total = npix * cv;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
-       i += (long long)gridDim.x * blockDim.x) {
-    const long long p = i / cv;
-    const int v = (int)(i % cv) * 8;
-    uint4* d = reinterpret_cast<uint4*>(dst + p * dst_c + dst_coff + v);
-    float a[8], t[8];
-    unpack8(*d, a);
-    unpack8(*reinterpret_cast<const uint4*>(src + p * src_c + src_coff + v), t);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) a[j] += t[j];
-    *d = pack8(a);
-  }
-}
-__global__ void add_f32_kernel(float* __restrict__ dst, const float* __restrict__ src, long long n) {
-  pdl_trigger();
-  pdl_wait();
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-       i += (long long)gridDim.x * blockDim.x)
-    dst[i] += src[i];
-}
-
 // grid such that (grid*256) % vec_per_pix == 0 so each thread keeps one channel lane
 inline int bn_grid(long long npix, int c, int per_thread, int max_blocks = 148 * 8) {
   const int vpp = c / 8;
@@ -576,35 +538,18 @@ typedef __nv_bfloat16 bf16;
 
 extern "C" {
 
-static int bn_stats_launch(const void* z, float* stats, float* mean_invstd, float* running_mean, float* running_var,
-                           int64_t npix, int32_t c, float momentum, float eps, b200_stream_t stream) {
-  B200_REQUIRE(c % 8 == 0 && c <= 2048 && 256 % (c / 8) == 0, "b200_bn_stats: c/8 must be a power of two <= 256 (c=%d)", c);
+int b200_bn_stats_finalize(const void* z, float* stats, float* mean_invstd, float* running_mean,
+                           float* running_var, int64_t npix, int32_t c, float momentum, float eps,
+                           b200_stream_t stream) {
+  B200_REQUIRE(mean_invstd != nullptr, "b200_bn_stats_finalize: mean_invstd is required");
+  B200_REQUIRE(c % 8 == 0 && c <= 2048 && 256 % (c / 8) == 0,
+               "b200_bn_stats_finalize: c/8 must be a power of two <= 256 (c=%d)", c);
   const int grid = bn_grid(npix, c, 4, 148 * 2);   // the last block adds the per-block partials: keep them few
   DetScratch ds;
   if (det_scratch(&ds, (size_t)(grid + det_groups(grid)) * 2 * c, 1 + det_groups(grid))) return 1;
   ::b200::launch_kernel(bn_reduce_kernel<0>, grid, 256, 16 * 256 * sizeof(float), as_stream(stream),
       (const bf16*)z, nullptr, nullptr, nullptr, nullptr, stats, (long long)npix, c, 0.f, ds.part, ds.counters, nullptr, nullptr,
       mean_invstd, running_mean, running_var, momentum, eps);
-  B200_LAUNCH_CHECK();
-  return 0;
-}
-
-int b200_bn_stats(const void* z, float* stats, int64_t npix, int32_t c, b200_stream_t stream) {
-  return bn_stats_launch(z, stats, nullptr, nullptr, nullptr, npix, c, 0.f, 0.f, stream);
-}
-
-int b200_bn_stats_finalize(const void* z, float* stats, float* mean_invstd, float* running_mean,
-                           float* running_var, int64_t npix, int32_t c, float momentum, float eps,
-                           b200_stream_t stream) {
-  B200_REQUIRE(mean_invstd != nullptr, "b200_bn_stats_finalize: mean_invstd is required");
-  return bn_stats_launch(z, stats, mean_invstd, running_mean, running_var, npix, c, momentum, eps, stream);
-}
-
-int b200_bn_finalize(const float* stats, float* mean_invstd, float* running_mean,
-                     float* running_var, int64_t npix, int32_t c, float momentum, float eps,
-                     b200_stream_t stream) {
-  ::b200::launch_kernel(bn_finalize_kernel, (c + 127) / 128, 128, 0, as_stream(stream), 
-      stats, mean_invstd, running_mean, running_var, npix, c, momentum, eps);
   B200_LAUNCH_CHECK();
   return 0;
 }
@@ -754,22 +699,6 @@ int b200_nhwc_bf16_to_nchw_f32(const void* x, float* y, int32_t n, int32_t c, in
                                int32_t cx, int32_t x_coff, b200_stream_t stream) {
   ::b200::launch_kernel(nhwc_to_nchw_kernel, grid_for((long long)n * c * h * w, 256), 256, 0, as_stream(stream), 
       (const bf16*)x, y, n, c, h, w, cx, x_coff);
-  B200_LAUNCH_CHECK();
-  return 0;
-}
-
-int b200_add_slice_bf16(void* dst, int32_t dst_c, int32_t dst_coff, const void* src, int32_t src_c,
-                        int32_t src_coff, int64_t npix, int32_t c, b200_stream_t stream) {
-  B200_REQUIRE(c % 8 == 0 && dst_c % 8 == 0 && src_c % 8 == 0 && dst_coff % 8 == 0 && src_coff % 8 == 0,
-               "b200_add_slice_bf16: channels must be multiples of 8");
-  ::b200::launch_kernel(add_slice_kernel, grid_for(npix * (c / 8), 256), 256, 0, as_stream(stream), 
-      (bf16*)dst, dst_c, dst_coff, (const bf16*)src, src_c, src_coff, npix, c);
-  B200_LAUNCH_CHECK();
-  return 0;
-}
-
-int b200_add_f32(float* dst, const float* src, int64_t numel, b200_stream_t stream) {
-  ::b200::launch_kernel(add_f32_kernel, grid_for(numel, 256), 256, 0, as_stream(stream), dst, src, numel);
   B200_LAUNCH_CHECK();
   return 0;
 }

@@ -25,7 +25,8 @@
 //     swizzle phase: the row offset is 256), completing on the peer's mbarrier;
 //   * across cluster edges through L2 in "LL" form: every 16-byte store carries 8 bytes of data and two copies of a
 //     4-byte sequence flag (8-byte atomicity), the receiver polls the data itself -- no fence, no separate flag
-//     (the round-1 kernel rdb_persist.cu spent ~6.5 k cycles per stage on store -> fence -> flag -> acquire -> TMA).
+//     (a separate flag costs store -> fence -> flag -> acquire -> TMA, ~6.5 k cycles per stage in
+//     profiles/r01_rdb_persist_timeline.txt).
 //
 // The gather-form input gradient of a block has exactly the same shape with the slices taken in reverse
 // (dO, dY4 .. dY1 -> d(x4) .. d(x)), so the backward trunk is the same kernel with flipped taps.
@@ -64,7 +65,6 @@ struct ChainParams {
   int pos0, range_len, n_tiles;   // first position, positions and 256-position super-tiles of the image group
   int b_stages;            // weight ring slots in use
   int n_regions;           // operand regions in rotation (2, or 3 with split stages)
-  int mcast;               // multicast the stage weights to the cluster (one L2 read per cluster instead of per CTA)
   int split;               // issue every stage as (completing columns, later convs) -- see part_rows()
   int tap_sign;            // +1 forward taps, -1 input-gradient taps
   uint8_t* ll;             // LL exchange buffers [tile][side][parity][halo rows][256 B]
@@ -191,32 +191,6 @@ __device__ __forceinline__ void dsmem_push(uint32_t dst_cluster, uint32_t src_ct
                "r"(src_cta), "r"(bytes), "r"(mbar_cluster)
                : "memory");
 }
-// arrive on an mbarrier of a peer CTA (shared::cluster address)
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-  }
-}
-// TMA tile load delivered to the same shared-memory offset (and mbarrier) of every CTA in `mask`
-__device__ __forceinline__ void tma_load_3d_mcast(void* smem, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2,
-                                                  uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4, %5}], [%2], %6;" ::"r"(smem_u32(smem)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-      : "memory");
-}
-
 // A stage may be issued in two parts: part 0 = the 32 (j = 4: 64) accumulator columns that stage j COMPLETES, part 1 =
 // the columns of the later convs, so that the epilogue / halo exchange of the completed columns overlaps part 1 on the
 // tensor pipe (the N = 32 MMAs of part 0 are shared-memory-operand bound: the price of starting the turnaround early).
@@ -237,7 +211,7 @@ rdb_chain_kernel(const __grid_constant__ ChainParams p) {
       reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   // slice_ready[parity]: operand region `parity` complete = 8 epilogue warps (own rows, cluster-edge halos) + 1
   // expect_tx arrival covering the bytes the in-cluster neighbours push through distributed shared memory
-  __shared__ uint64_t b_full[kBStages], b_empty[kBStages], grp_empty[kBStages], init_full, slice_ready[3], acc_ready;
+  __shared__ uint64_t b_full[kBStages], b_empty[kBStages], init_full, slice_ready[3], acc_ready;
   __shared__ uint32_t tmem_base_s;
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
@@ -246,17 +220,8 @@ rdb_chain_kernel(const __grid_constant__ ChainParams p) {
   const int crank = p.cluster_size > 1 ? (int)cluster_ctarank() : 0;
   const bool active = cta < p.n_tiles;   // CTAs that only pad the grid to a multiple of the cluster size do nothing
   if (threadIdx.x == 0) {
-    // weight multicast: the active CTAs of a cluster (always a prefix of its ranks) consume identical weight tiles;
-    // the cluster's first CTA loads each tile ONCE from L2 and multicasts it, after every CTA reported the slot free
-    int grp_n = 1;
-    if (p.mcast) {
-      const int first = cta - crank;
-      grp_n = p.n_tiles - first < p.cluster_size ? p.n_tiles - first : p.cluster_size;
-      if (grp_n < 1) grp_n = 1;
-    }
     for (int s = 0; s < p.b_stages; ++s) {
       mbar_init(&b_full[s], 1);
-      mbar_init(&grp_empty[s], grp_n);
       mbar_init(&b_empty[s], 2);       // both MMA issuers
     }
     mbar_init(&init_full, 1);
@@ -307,12 +272,6 @@ rdb_chain_kernel(const __grid_constant__ ChainParams p) {
       __syncwarp();
       int bs = 0;
       uint32_t bph = 0;
-      uint16_t mcast_mask = 0;
-      if (p.mcast) {
-        const int first = cta - crank;
-        const int grp = p.n_tiles - first < p.cluster_size ? p.n_tiles - first : p.cluster_size;
-        mcast_mask = (uint16_t)((1u << grp) - 1u);
-      }
       for (int blk = 0; blk < p.n_blocks; ++blk) {
         for (int j = 0; j < 5; ++j) {
           for (int part = 0; part < 2; ++part) {
@@ -326,20 +285,9 @@ rdb_chain_kernel(const __grid_constant__ ChainParams p) {
               mbar_wait(&b_empty[bs], bph ^ 1);
               if (elect_one()) {
                 mbar_expect_tx(&b_full[bs], tap_bytes * nt);
-                if (!p.mcast) {
-                  for (int q = 0; q < nt; ++q)
-                    tma_load_3d(smem + b_ring_off + (size_t)bs * kBStageBytes + (size_t)q * tap_bytes, &p.w_map[j][part],
-                                &b_full[bs], 0, row0, blk * 9 + t0 + q);
-                } else {
-                  // slot free here and its barrier armed -> tell the cluster's first CTA; it loads once for everybody
-                  mbar_arrive_cluster(mapa_cluster(smem_u32(&grp_empty[bs]), 0u));
-                  if (crank == 0) {
-                    mbar_wait_cluster(&grp_empty[bs], bph);
-                    for (int q = 0; q < nt; ++q)
-                      tma_load_3d_mcast(smem + b_ring_off + (size_t)bs * kBStageBytes + (size_t)q * tap_bytes,
-                                        &p.w_map[j][part], &b_full[bs], 0, row0, blk * 9 + t0 + q, mcast_mask);
-                  }
-                }
+                for (int q = 0; q < nt; ++q)
+                  tma_load_3d(smem + b_ring_off + (size_t)bs * kBStageBytes + (size_t)q * tap_bytes, &p.w_map[j][part],
+                              &b_full[bs], 0, row0, blk * 9 + t0 + q);
               }
               __syncwarp();
               if (++bs == p.b_stages) {
@@ -648,17 +596,10 @@ extern "C" int b200_rdb_chain(const b200_chain_desc* d, const void* x0, const vo
   p.box_rows = (((region + p.nbox - 1) / p.nbox) + 7) & ~7;
   p.a_bytes = (uint32_t)p.nbox * p.box_rows * 128;
   p.a_region_bytes = (p.a_bytes + 1023) & ~1023u;
-  {
-    static int split = -1;
-    if (split < 0) {
-      const char* e = getenv("B200_CHAIN_SPLIT");
-      split = e ? atoi(e) : 1;
-    }
-    p.split = split ? 1 : 0;
-  }
-  p.n_regions = p.split ? 3 : 2;
+  p.split = 1;
+  p.n_regions = 3;
   int b_stages = (227 * 1024 - 1024 - p.n_regions * (int)p.a_region_bytes) / (int)kBStageBytes;
-  if (b_stages < 3 && p.split) {   // not enough room for three regions: one-piece stages with two
+  if (b_stages < 3) {   // not enough room for three regions (w >= 70): one-piece stages with two
     p.split = 0;
     p.n_regions = 2;
     b_stages = (227 * 1024 - 1024 - 2 * (int)p.a_region_bytes) / (int)kBStageBytes;
@@ -713,14 +654,7 @@ extern "C" int b200_rdb_chain(const b200_chain_desc* d, const void* x0, const vo
   }
   // Thread-block clusters: neighbouring tiles inside a cluster exchange their halo rows through distributed
   // shared memory (bulk copy + remote mbarrier), only the cluster-edge halos go through L2.  The largest cluster
-  // size (<= B200_CHAIN_CLUSTER, default 8) whose clusters are all co-resident is used.
-  static int cs_max = -1;
-  if (cs_max < 0) {
-    const char* e = getenv("B200_CHAIN_CLUSTER");
-    cs_max = e ? atoi(e) : 8;
-    if (cs_max < 1) cs_max = 1;
-    if (cs_max > 8) cs_max = 8;
-  }
+  // size (<= 8, the portable maximum) whose clusters are all co-resident is used.
   int cs = 1, grid = n_cta;
   // decided once per grid size (the occupancy query must not run inside a stream capture)
   static std::mutex cs_mu;
@@ -735,7 +669,7 @@ extern "C" int b200_rdb_chain(const b200_chain_desc* d, const void* x0, const vo
       cached = true;
     }
   }
-  for (int c = cached ? 0 : cs_max; c >= 2; --c) {   // any size, not only powers of two: 6 fits where 4 + 4 + .. does not
+  for (int c = cached ? 0 : 8; c >= 2; --c) {   // any size, not only powers of two: 6 fits where 4 + 4 + .. does not
     const int g = (n_cta + c - 1) / c * c;
     cudaLaunchConfig_t q = {};
     q.gridDim = dim3(g);
@@ -767,14 +701,6 @@ extern "C" int b200_rdb_chain(const b200_chain_desc* d, const void* x0, const vo
     cs_cache[n_cta] = cs;
   }
   p.cluster_size = cs;
-  {
-    static int mc = -1;
-    if (mc < 0) {
-      const char* e = getenv("B200_CHAIN_MCAST");
-      mc = e ? atoi(e) : 0;   // opt-in: measured SLOWER (4.93 vs 4.82 ms): one CTA issuing the cluster's loads + a per-slot handshake
-    }
-    p.mcast = (mc && cs > 1) ? 1 : 0;
-  }
   ::b200::launch_kernel(chain_epoch_bump_kernel, 1, 1, 0, as_stream(stream), epoch_dev);
   B200_LAUNCH_CHECK();
   cudaLaunchConfig_t cfg = {};

@@ -18,8 +18,6 @@
 // element is owned by exactly one item), then `+=` into the fp32 OIHW gradient tensors.
 //
 // Reference: autograd wgrad of the 5 convs of ResidualDenseBlock_5C (RRDBNet_arch.py:130-148).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "colsum.cuh"
 #include "sm100_ptx.cuh"
@@ -384,14 +382,9 @@ namespace {
 // writes its own tap-major slab of the caller's workspace with plain coalesced stores and a second kernel adds
 // the slabs in slice order: deterministic (round 1 used fp32 atomics: S=1 3.76 ms, S=4 3.41 ms, S=8 4.32 ms
 // because of the exposed atomic epilogue; operand phase alone 2.55 ms for S >= 4).
+constexpr int kSplit = 4;   // measured (deterministic slabs): S=1 3.76 ms, S=4 3.31 ms, S=8 4.09 ms
 void rdb_split(int k_steps, int* k_split, int* k_per) {
-  static int ksplit_env = -1;
-  if (ksplit_env < 0) {
-    const char* e = getenv("B200_WGRAD_RDB_KSPLIT");
-    ksplit_env = e ? atoi(e) : 4;   // measured (deterministic slabs): S=1 3.76 ms, S=4 3.31 ms, S=8 4.09 ms
-    if (ksplit_env < 1) ksplit_env = 1;
-  }
-  int s = ksplit_env < k_steps ? ksplit_env : 1;
+  int s = kSplit < k_steps ? kSplit : 1;
   *k_per = (k_steps + s - 1) / s;
   *k_split = (k_steps + *k_per - 1) / *k_per;   // no empty slices
 }

@@ -7,7 +7,6 @@ Only Z is kept for backward (the activation and its LeakyReLU mask are recompute
 batch statistics).  Every train-mode forward updates running_mean / running_var /
 num_batches_tracked exactly like nn.BatchNorm2d (4 updates per training iteration, SURVEY 7.5).
 """
-import os
 import weakref
 
 import torch
@@ -35,9 +34,6 @@ class DiscriminatorEngine:
         # optimizer (models/sr_model.py) switches it on.
         self.reuse = False
         self._cache = {}
-        # BatchNorm batch statistics from the conv epilogue where the conv kernel offers it (B200_BN_FUSE_STATS=0:
-        # always a separate pass over the conv output)
-        self.fuse_stats = os.environ.get("B200_BN_FUSE_STATS", "1") != "0"
 
     def _setup(self, device):
         net = self.net
@@ -95,9 +91,10 @@ class DiscriminatorEngine:
                 d = make_conv_desc(N, hi, hi, L.cin, 0, L.cin, ho, ho, ho, ho, L.cout, 0, L.cout,
                                    taps_conv(L.kh, L.pad), L.taps, L.fwd_rows, L.fwd_cols, in_stride=L.stride)
                 npix = N * ho * ho
-                rows = igemm_stat_rows(d) if (train and self.fuse_stats) else 0
+                rows = igemm_stat_rows(d) if train else 0
                 if rows:
-                    # batch statistics from the conv epilogue (per-tile partial sums) instead of a pass over Z
+                    # batch statistics from the conv epilogue (per-tile partial sums) where the conv kernel offers it,
+                    # instead of a pass over Z
                     if ctx.stat_part[i] is None:
                         ctx.stat_part[i] = torch.empty(2 * L.cout * rows, dtype=torch.float32, device=dev)
                     add_igemm_stats(f, d, ctx.A[i], L.w_fwd, L.bias, ctx.Z[i], ctx.stat_part[i])

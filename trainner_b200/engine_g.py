@@ -19,7 +19,7 @@ import os
 import torch
 
 from . import _lib
-from ._lib import ChainDesc, ChainStage, ColsumEntry, PackCatEntry, RdbDesc, WgradRdbEntry, lib
+from ._lib import ChainDesc, ChainStage, ColsumEntry, PackCatEntry, WgradRdbEntry, lib
 from .runtime import sm_count_hint
 from .runtime import (ConvLayer, ContextPool, pool_for, FlatGrads, Lease, LRELU_SLOPE, P, Plan, WeightPacker,
                       add_flat, add_igemm, add_wgrad, make_conv_desc, make_flat_desc, require_device, taps_conv,
@@ -79,26 +79,19 @@ class RRDBNetEngine:
                                                 k1p, a, 0, 1, 0))
                 per_slice.append((wt, n_s, lo, k1, cols))
             self.wcat.append(per_slice)
-        # TMEM-persistent stage-merged dense block (csrc/rdb_persist.cu): stage weights
+        # Whole-trunk chain (csrc/rdb_chain.cu): stage-merged dense blocks with the slices kept in shared memory
+        # and ONE launch per image group for all dense blocks -- the default trunk path (B200_TRUNK_CHAIN=0: the
+        # per-conv flat kernels).  Shapes it does not cover (w > 125, nf != 64, gc != 32) use the flat kernels.
         #   forward  stage j: rows = outputs of conv_{j+1}..conv5 (192-32j), cols = the stage's input slice
         #   backward stage j: rows = slices x_{4-j}..x (TMEM column order), cols = dY of conv_{5-j}
-        # Opt-in (B200_RDB_PERSIST=1): numerically verified, but its 5-stage neighbour-sync latency chain
-        # (~10k cycles/stage vs ~3.5k cycles of MMA; profiles/r01_rdb_persist_timeline.txt) makes it no
-        # faster than the flat per-conv kernels at 16 images/GPU, so the flat path stays the default.
-        self.persist = os.environ.get("B200_RDB_PERSIST", "0") == "1"
-        # Whole-trunk chain (csrc/rdb_chain.cu): the same stage-merged form with the slices kept in shared memory
-        # and ONE launch per image group for all dense blocks -- the default trunk path (B200_TRUNK_CHAIN=0: the
-        # per-conv flat kernels).  Shapes it does not cover (w > 128, nf != 64, gc != 32) use the flat kernels.
-        self.chain = os.environ.get("B200_TRUNK_CHAIN", "1") == "1" and nf == 64 and gc == 32 and not self.persist
-        self.wstage_f, self.wstage_b = [], []
+        self.chain = os.environ.get("B200_TRUNK_CHAIN", "1") == "1" and nf == 64 and gc == 32
         nrdb_ = len(self.rdbs)
-        if self.persist or self.chain:
+        if self.chain:
             # stage weights of all blocks, contiguous per stage: WF[j][r], WB[j][nrdb-1-r] (chain order of the backward)
             self.WF = [torch.zeros(nrdb_, 9, 192 - 32 * j, nf if j == 0 else gc, dtype=BF16, device=device) for j in range(5)]
             self.WB = [torch.zeros(nrdb_, 9, 192 - 32 * j, nf if j == 0 else gc, dtype=BF16, device=device) for j in range(5)]
             for r, convs in enumerate(self.rdbs):
                 a = 0.04 if r % 3 == 2 else 0.2
-                wf, wb = [], []
                 for j in range(5):
                     n_j = 192 - 32 * j
                     kc = nf if j == 0 else gc   # stage input channels = packed K width (64 or 32)
@@ -114,10 +107,6 @@ class RRDBNetEngine:
                         so, sn = (nf + (3 - sp) * gc, gc) if sp < 4 else (0, nf)
                         cat_entries.append(PackCatEntry(cv.weight.data_ptr(), tb.data_ptr(), cv.cout, cv.cin, 9, so, sn,
                                                         n_j, kc, 0, a if j == 0 else 1.0, gc * (sp - j), 1, 0))
-                    wf.append(tf)
-                    wb.append(tb)
-                self.wstage_f.append(wf)
-                self.wstage_b.append(wb)
         self.packer = WeightPacker(self.tc_layers, device, cat_entries)
         self.grads = FlatGrads(list(net.parameters()), device)
         self.pools = {}
@@ -126,16 +115,6 @@ class RRDBNetEngine:
         require_device(x, "RRDBNet")
         if self.device != x.device or self.packer.stale_pointers():
             self._setup(x.device)
-
-    def _image_groups(self, N, h, w):
-        """image ranges whose flat positions fit one 256-row tile per SM (rdb_persist is one tile per CTA)"""
-        per = (h + 2) * (w + 2)
-        g = max(1, (sm_count_hint() * 256) // per)
-        if g * per > sm_count_hint() * 256:
-            g -= 1
-        if g < 1:
-            raise RuntimeError("RRDBNet: image too large for the persistent dense-block kernel")
-        return [(i, min(g, N - i)) for i in range(0, N, g)]
 
     @staticmethod
     def _chain_geometry(n, h, w):
@@ -193,10 +172,7 @@ class RRDBNetEngine:
         f.add(lib.b200_conv3x3_thin_to_wide, P(ctx.x), P(self.fea.weight), P(self.fea.bias), P(ctx.F0),
               N, h, w, net.in_nc, nf, nf, 0, 0, None, None, 0, 0.0, None, 0, 0, 0.0)
         f.add(lib.b200_pad_copy, P(ctx.B[0]), Bc[0], 0, P(ctx.F0), nf, 0, N, h, w, nf)
-        groups = self._image_groups(N, h, w) if self.persist else []
-        ctx.flags = torch.zeros(256, dtype=torch.int32, device=dev) if self.persist else None
-        use_chain = self.chain
-        ctx.chain_groups = self._chain_groups(N, h, w) if use_chain else None
+        ctx.chain_groups = self._chain_groups(N, h, w) if self.chain else None
         use_chain = ctx.chain_groups is not None
         if use_chain:
             ll_bytes = max(self._chain_geometry(gn, h, w)[1] for _, gn in ctx.chain_groups)
@@ -233,31 +209,6 @@ class RRDBNetEngine:
             last_of_rrdb = (r % 3 == 2)
             a = 0.04 if last_of_rrdb else 0.2
             b1 = 0.2 if last_of_rrdb else 1.0
-            if self.persist:
-                for (g0, gn) in groups:
-                    d = RdbDesc()
-                    d.n, d.h, d.w = gn, h, w
-                    bi, bo = Bi[g0:g0 + gn], Bo[g0:g0 + gn]
-                    for j in range(5):
-                        st = d.stage[j]
-                        st.x, st.cx = bi.data_ptr(), C
-                        st.cin_off, st.cin = (0, nf) if j == 0 else (nf + (j - 1) * gc, gc)
-                        st.w_packed = self.wstage_f[r][j].data_ptr()
-                        st.bias = convs[j].bias.data_ptr()
-                        st.alpha, st.slope = 1.0, LRELU_SLOPE
-                        if j < 4:
-                            st.out, st.out_c, st.out_coff, st.act = bi.data_ptr(), C, nf + j * gc, 1
-                        else:
-                            st.out, st.out_c, st.out_coff, st.act = bo.data_ptr(), Bc[r + 1], 0, 0
-                            st.alpha = a
-                            st.res1, st.res1_c, st.res1_coff, st.beta1 = bi.data_ptr(), C, 0, b1
-                            if last_of_rrdb:
-                                st.res2, st.res2_c, st.res2_coff, st.beta2 = ctx.B[r - 2][g0:g0 + gn].data_ptr(), C, 0, 1.0
-                    f.keep(d)
-                    f.add(lib.b200_rdb_persist, CT.byref(d), P(ctx.flags), 0,
-                          flops=2.0 * gn * h * w * 9 * (nf * gc + (nf + gc) * gc + (nf + 2 * gc) * gc + (nf + 3 * gc) * gc + C * nf),
-                          tag="rdb_persist", info="fwd %d img" % gn)
-                continue
             for kk in range(4):
                 L = convs[kk]
                 cin = nf + kk * gc
@@ -415,33 +366,6 @@ class RRDBNetEngine:
             first_of_rrdb = (r % 3 == 0)
             a = 0.04 if last_of_rrdb else 0.2
             b1 = 0.2 if last_of_rrdb else 1.0
-            if self.persist:
-                for (g0, gn) in self._image_groups(N, h, w):
-                    d = RdbDesc()
-                    d.n, d.h, d.w, d.flip_taps = gn, h, w, 1
-                    gr, do_, br = Gr[g0:g0 + gn], dO[g0:g0 + gn], Br[g0:g0 + gn]
-                    for j in range(5):
-                        st = d.stage[j]
-                        if j == 0:
-                            st.x, st.cx, st.cin_off, st.cin = do_.data_ptr(), CC, 0, nf
-                        else:
-                            st.x, st.cx, st.cin_off, st.cin = gr.data_ptr(), CC, nf + (4 - j) * gc, gc
-                        st.w_packed = self.wstage_b[r][j].data_ptr()
-                        st.alpha, st.mask_slope = 1.0, SL
-                        st.out, st.out_c = gr.data_ptr(), CC
-                        if j < 4:
-                            st.out_coff = nf + (3 - j) * gc
-                            st.mask, st.mask_c, st.mask_coff = br.data_ptr(), CC, nf + (3 - j) * gc
-                        else:
-                            st.out_coff = 0
-                            st.res1, st.res1_c, st.res1_coff, st.beta1 = do_.data_ptr(), CC, 0, b1
-                            if first_of_rrdb:
-                                st.res2, st.res2_c, st.res2_coff, st.beta2 = slot(r + 3)[g0:g0 + gn].data_ptr(), CC, 0, 1.0
-                    b.keep(d)
-                    b.add(lib.b200_rdb_persist, CT.byref(d), P(ctx.flags), 0,
-                          flops=2.0 * gn * h * w * 9 * (nf * gc + (nf + gc) * gc + (nf + 2 * gc) * gc + (nf + 3 * gc) * gc + CC * nf),
-                          tag="rdb_persist", info="bwd %d img" % gn)
-                continue
             for sl in range(4, -1, -1):
                 wt, n_s, lo, k1, cols = self.wcat[r][sl]
                 kw = dict(cx2=CC, cin2_off=0, cin2=nf)
